@@ -64,7 +64,15 @@ def parse():
     ap.add_argument("--out", default="")
     ap.add_argument("--max-bytes", type=int, default=1 << 30)
     ap.add_argument("--region-mb", type=int, default=1024)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="allreduce mode: after the timed steps write the all-reduced gradients of the last step "
+                         "as DIR/grad_<i>.npy (float64, a fixed seeded sample of each tensor, under 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "allreduce" or args.impl != "ours"):
+        ap.error("--dump-outputs needs --mode allreduce --impl ours")
+    return args
 
 
 def reference_arm(args):
@@ -253,6 +261,26 @@ def load_tuning(comm, args, dist):
         return None
 
 
+def dump_outputs(out_dir, views, budget_bytes=48 << 20, seed=0):
+    """Write each tensor of `views` as float64 (exact for int32) to
+    out_dir/grad_<i>.npy.  When the whole set exceeds `budget_bytes`, every
+    tensor is cut to the same fraction of its elements, picked by a fixed seed
+    and kept in index order, so that runs of two builds compare element for element."""
+    import numpy as np
+    import torch
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    frac = min(1.0, budget_bytes / 8 / sum(v.numel() for v in views))
+    gen = torch.Generator().manual_seed(seed)
+    for i, v in enumerate(views):
+        n = v.numel()
+        k = max(1, int(n * frac))
+        if k < n:
+            v = v[torch.randperm(n, generator=gen)[:k].sort().values.to(v.device)]
+        np.save(out / f"grad_{i:03d}.npy", v.to(torch.float64).cpu().numpy())
+
+
 def peaks():
     p = ROOT / "MEASURED_PEAKS.json"
     if p.exists():
@@ -325,6 +353,8 @@ def mode_allreduce(args, dist: Dist):
         sampler = ClockSampler(gpu_index=dist.local).start() if dist.rank == 0 else None
         ms = timed(dist, sync.step, args.steps, args.warmup)
         clocks = sampler.stop() if sampler else {}
+        if args.dump_outputs and dist.rank == 0:
+            dump_outputs(args.dump_outputs, sync.recv_views)
         launches = sync.launches_per_step * args.steps
         err = comm.check_error()
         if err:
@@ -703,7 +733,7 @@ def mode_threads(args, dist: Dist):
     return out, {}
 
 
-def mpi_api_arm(n: int) -> dict:
+def mpi_api_arm(n: int, steps: int, warmup: int) -> dict:
     """Runs `bench.py --impl mpi-symmetric-nb` in a child (its own worker process with n rank threads)."""
     import subprocess
 
@@ -712,7 +742,7 @@ def mpi_api_arm(n: int) -> dict:
                         "MASTER_PORT", "TORCHELASTIC_RUN_ID")}
     try:
         r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "mpi-symmetric-nb", "--gpus", str(n),
-                            "--steps", "10", "--warmup", "3"], capture_output=True, text=True, timeout=300, env=env)
+                            "--steps", str(steps), "--warmup", str(warmup)], capture_output=True, text=True, timeout=300, env=env)
         res = json.loads(r.stdout.strip().splitlines()[-1])
         return {"impl": "MPI_Iallreduce x214 + MPI_Waitall (C API, symmetric device memory)", "world_size": res["world_size"],
                 "ms_per_step": res["ms_per_step"], "us_per_allreduce": round(res["ms_per_step"] * 1000 / res["config"]["tensors"], 3),
@@ -753,7 +783,7 @@ def main():
         keep = None
         dist.torch.cuda.synchronize()
         if dist.rank == 0:
-            out["mpi_api"] = mpi_api_arm(max(dist.world, 2))
+            out["mpi_api"] = mpi_api_arm(max(dist.world, 2), args.steps, args.warmup)
     if dist.rank == 0:
         line = json.dumps(out)
         print(line, flush=True)

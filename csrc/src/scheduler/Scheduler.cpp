@@ -60,9 +60,12 @@ void Scheduler::addHostToGlobalSet(
         req->mutable_host()->set_usedslots(overwriteResources->usedslots());
         req->set_overwrite(true);
     } else if (hostIp == thisHost) {
-        // Execution slots: CPU cores, or slots-per-GPU x GPUs on a GPU box
+        // Execution slots: CPU cores, or slots-per-GPU x GPUs on a GPU box.
+        // OVERRIDE_CPU_COUNT wins on both, as it also sizes the executor's
+        // thread pool
         int gpus = faabric::util::getUsableGpus();
-        int slots = gpus > 0 ? gpus * conf.slotsPerGpu : (int)faabric::util::getUsableCores();
+        int slots = (conf.overrideCpuCount > 0 || gpus == 0) ? (int)faabric::util::getUsableCores()
+                                                             : gpus * conf.slotsPerGpu;
         req->mutable_host()->set_slots(slots);
         req->mutable_host()->set_usedslots(0);
     }
